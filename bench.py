@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- generations/sec of the ES hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one ES generation (estorch.py:214-248): evaluate the P = 4096 mirrored members of the
@@ -16,6 +16,10 @@ sum_j w_j * noise_j, negate/clamp, Adam, post-update rollout.  Prints ONE JSON l
   roofline / kernels   per-kernel achieved rate vs MEASURED_PEAKS.json
   cpu_baseline         the reference's CPU path on this box's host cores, bounded sample, rank 0 / N=1
   extra                the other BASELINE.json configs through the same public API (short runs)
+
+`--dump-outputs DIR` writes, after the timed generations, what a caller of ES.train holds after the last
+one (parameters, population returns, episode / best reward, best policy) as DIR/<name>.npy; the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` runs only the reference's CPU path (rank 0): the UNMODIFIED reference package from
 baseline/_ref (installed by __graft_entry__.build()) when present, else the CPU port of its cost
@@ -278,6 +282,32 @@ def build_es(wl, args, eval_precision, log_interval):
     return es, obs, tgt
 
 
+def capture_outputs(es):
+    """What a caller of ES.train holds after the last generation, copied to the host (float32 arrays,
+    float64 scalars)."""
+    def flat(module):
+        return torch.nn.utils.parameters_to_vector(module.parameters()).detach().float().cpu().numpy()
+    out = {"population_returns": np.array(es.population_returns, dtype=np.float32),      # a copy: the host cache is reused
+           "episode_reward": np.array([es.episode_reward], dtype=np.float64),
+           "best_reward": np.array([es.best_reward], dtype=np.float64),
+           "best_policy": np.concatenate([v.detach().float().cpu().reshape(-1).numpy()
+                                          for v in es.best_policy_dict.values()])}
+    if hasattr(es, "meta_population"):
+        out["meta_population"] = np.stack([flat(policy) for policy, _ in es.meta_population])
+    else:
+        out["policy"] = flat(es.policy)
+    return out
+
+
+def dump_outputs(outputs, directory, limit=64 << 20):
+    total = sum(a.nbytes for a in outputs.values())
+    if total > limit:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {limit}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def timed_region(es, steps, warmup, world, dev, sampler=None):
     """(ms, wall s, clocks, launches) of `steps` generations: CUDA events around the region,
     barrier + synchronize on both sides, max over ranks."""
@@ -337,6 +367,7 @@ def run_ours(args, wl, rank, world, local_rank):
     # ---- value: device-resident, no host sync in the loop
     sampler = ClockSampler(local_rank) if rank == 0 else None   # nvidia-smi needs ~1 s to start streaming
     ms, _, clocks, launches = timed_region(es, args.steps, args.warmup, world, dev, sampler)
+    outputs = capture_outputs(es) if args.dump_outputs and rank == 0 else None
 
     # ---- e2e: host buffers in, log() + host results out, every generation
     es.agent.stream_from_host, es.read_back, es._log_interval = True, True, 1
@@ -368,6 +399,8 @@ def run_ours(args, wl, rank, world, local_rank):
 
     if rank != 0:
         return
+    if outputs is not None:
+        dump_outputs(outputs, args.dump_outputs)
     line = {"metric": METRIC, "value": args.steps / (ms / 1e3),
             "unit": "generations/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": ms / args.steps, "higher_is_better": True, "scaling": "strong",
@@ -511,6 +544,7 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the short runs of the other BASELINE configs")
     ap.add_argument("--extras", default="", help="comma list of other workloads to run in the same process (any N)")
     ap.add_argument("--eval-precision", default="auto", choices=["auto", "fp32", "f16", "bf16", "bf16s"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed generation's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     # >= 5 warm-up generations on our arm: a generation configuration is captured into a CUDA graph at its third
     # sighting, so the capture (tens of ms) happens in the warm-up, never inside the timed region

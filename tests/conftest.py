@@ -18,6 +18,15 @@ def load_golden(name):
     return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
 
 
+def seeded_theta(g):
+    """Parameter vector of a fixture that stores how to draw it rather than its values (large parameter
+    vectors would push a fixture past 1 MB): segment i is ``theta_sizes[i]`` draws from
+    U(theta_lo[i], theta_hi[i]) of ``np.random.RandomState(theta_seed)``, rounded to fp16."""
+    rng = np.random.RandomState(int(g["theta_seed"]))
+    parts = [rng.uniform(lo, hi, int(n)) for n, lo, hi in zip(g["theta_sizes"], g["theta_lo"], g["theta_hi"])]
+    return np.concatenate(parts).astype(np.float16).astype(np.float32)
+
+
 @pytest.fixture
 def golden():
     return load_golden

@@ -24,6 +24,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))     # tests/: conftest.seeded_theta
 
 
 def _install_shims():
@@ -169,6 +170,34 @@ def run_reference(cls, dims, P, sigma, n_gen, table, noise_seed, obs, target,
     return out
 
 
+def write_atari_fixture():
+    """Atari conv + VBN policy forward (examples/atari.py:14-37).  The 677k parameters are stored as the
+    recipe of conftest.seeded_theta (default-init ranges, gamma/beta spread around 1/0), not as values,
+    to keep the fixture small; frames are stored as uint8."""
+    import atari as ref_atari  # the reference example module (gym/skimage shimmed)
+    from conftest import seeded_theta
+    recipe = dict(theta_seed=2024, theta_sizes=[], theta_lo=[], theta_hi=[])
+    fan_in = 1
+    for name, shape in orc.atari_param_layout(4):
+        if name.endswith(".w") and len(shape) > 1:
+            fan_in = int(np.prod(shape[1:]))
+        lo, hi = (0.8, 1.2) if name.startswith("bn") and name.endswith(".w") else \
+            (-0.2, 0.2) if name.startswith("bn") else (-fan_in ** -0.5, fan_in ** -0.5)
+        recipe["theta_sizes"].append(int(np.prod(shape)))
+        recipe["theta_lo"].append(lo)
+        recipe["theta_hi"].append(hi)
+    recipe = {k: np.array(v) for k, v in recipe.items()}
+    g = torch.Generator().manual_seed(4321)
+    xref8 = (torch.rand(8, 4, 84, 84, generator=g) * 255).round().to(torch.uint8)
+    x8 = (torch.rand(3, 4, 84, 84, generator=g) * 255).round().to(torch.uint8)
+    pol = ref_atari.Policy(4, xref8.float() / 255)
+    torch.nn.utils.vector_to_parameters(torch.from_numpy(seeded_theta(recipe)), pol.parameters())
+    with torch.no_grad():
+        logits = pol(x8.float() / 255)
+    np.savez_compressed(os.path.join(HERE, "atari_forward.npz"), xref8=xref8.numpy(), x8=x8.numpy(),
+                        logits=logits.numpy(), **recipe)
+
+
 def main():
     # --- the one known-answer vector the reference ships (estorch.py:31-35) ---
     doc_in = np.array([-123, -50, 3, -5, 20, 10, 100], dtype=np.float64)
@@ -226,33 +255,7 @@ def main():
                         gamma=vbn.weight.detach().numpy(), beta=vbn.bias.detach().numpy(),
                         y_ref=y_ref.numpy(), y=y.numpy())
 
-    # --- Atari conv + VBN policy forward (examples/atari.py:14-37) ---
-    import atari as ref_atari  # the reference example module (gym/skimage shimmed)
-    torch.manual_seed(3)
-    xref = torch.rand(8, 4, 84, 84, generator=g)
-    pol = ref_atari.Policy(4, xref)
-    with torch.no_grad():
-        for p_ in pol.parameters():          # make gamma/beta non-trivial
-            if p_.dim() == 1:
-                p_.add_(0.1 * torch.randn(p_.shape, generator=g))
-        x = torch.rand(3, 4, 84, 84, generator=g)
-        logits = pol(x)
-    flat = _flat(pol.parameters())
-    np.savez_compressed(os.path.join(HERE, "atari_forward.npz"),
-                        theta=flat.astype(np.float16).astype(np.float32),  # placeholder, replaced below
-                        )
-    # store params at fp16 precision to keep the fixture small; recompute the
-    # reference output on exactly those rounded params
-    flat16 = flat.astype(np.float16).astype(np.float32)
-    torch.nn.utils.vector_to_parameters(torch.from_numpy(flat16), pol.parameters())
-    xref8 = (xref * 255).round().to(torch.uint8)
-    x8 = (x * 255).round().to(torch.uint8)
-    pol.xref = xref8.float() / 255
-    with torch.no_grad():
-        logits = pol(x8.float() / 255)
-    np.savez_compressed(os.path.join(HERE, "atari_forward.npz"),
-                        theta16=flat16.astype(np.float16), xref8=xref8.numpy(), x8=x8.numpy(),
-                        logits=logits.numpy())
+    write_atari_fixture()
     print("fixtures written to", HERE)
     for f in sorted(os.listdir(HERE)):
         if f.endswith(".npz"):

@@ -10,7 +10,7 @@ import pytest
 import torch
 
 from oracle import es_oracle as orc
-from conftest import load_golden, rel_err
+from conftest import load_golden, rel_err, seeded_theta
 
 pytestmark = pytest.mark.gpu
 
@@ -672,7 +672,7 @@ def test_eval_conv_vbn_matches_oracle_and_reference_golden(be):
     """examples/atari.py policy: (1) the centre evaluation reproduces the logits-based
     return of the reference's own forward (golden), (2) perturbed members match the oracle."""
     g = load_golden("atari_forward.npz")
-    theta = g["theta16"].astype(np.float32)
+    theta = seeded_theta(g)
     xref = g["xref8"].astype(np.float32) / np.float32(255)
     x = g["x8"].astype(np.float32) / np.float32(255)
     A, R, B = 4, xref.shape[0], x.shape[0]

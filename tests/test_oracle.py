@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from oracle import es_oracle as orc
-from conftest import load_golden, rel_err
+from conftest import load_golden, rel_err, seeded_theta
 
 
 def test_rank_docstring_vector():
@@ -133,7 +133,7 @@ def test_vbn_matches_reference():
 
 def test_atari_forward_matches_reference():
     g = load_golden("atari_forward.npz")
-    theta = g["theta16"].astype(np.float32)
+    theta = seeded_theta(g)
     xref = g["xref8"].astype(np.float32) / np.float32(255)
     x = g["x8"].astype(np.float32) / np.float32(255)
     logits = orc.atari_forward(theta, 4, xref, x)

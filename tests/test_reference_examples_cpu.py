@@ -1,15 +1,13 @@
-"""Drop-in check: the reference's own example scripts run against this package.
+"""Drop-in check: user programs written against the original estorch API run unchanged on this package.
 
-The scripts are READ at test time from /root/reference/examples (never copied into the
-repo; the tests skip where the reference is not mounted, e.g. on the GPU box).  They are
-executed with ``import estorch`` resolving to ``estorch_b200``, a stand-in ``gym`` (the image
-has no gym) and the CPU stand-in backend of tests/_oracle_backend.py.  Only the launch
-parameters are rewritten (``n_proc=2`` would re-exec under torchrun, hundreds of steps
-are cut to a few) -- the classes, hooks and attribute accesses are the reference's text.
+The programs below are the four usage patterns of the original project's example scripts
+(examples/cartpole_es.py, early_stopping.py, custom_es.py, nsra_es.py): the same classes, constructor
+arguments, overridden hooks and attribute accesses, at test size (``n_proc=1``, a few generations,
+population 8).  They ``import estorch``, which resolves to ``estorch_b200``, see a stand-in ``gym``
+(gym is not a dependency) and run on the CPU stand-in backend of tests/_oracle_backend.py.
 """
+import collections
 import math
-import os
-import re
 import sys
 import types
 
@@ -19,9 +17,6 @@ import torch
 
 import estorch_b200
 from _oracle_backend import OracleBackend
-
-EXAMPLES = "/root/reference/examples"
-pytestmark = pytest.mark.skipif(not os.path.isdir(EXAMPLES), reason="reference examples are not mounted here")
 
 
 class _Space:
@@ -87,16 +82,162 @@ class WalkerStandIn:
         pass
 
 
+
+
+class Policy(torch.nn.Module):
+    """The examples' policy: two hidden layers of 64 with ReLU."""
+
+    def __init__(self, n_input, n_output):
+        super().__init__()
+        self.linear_1 = torch.nn.Linear(n_input, 64)
+        self.linear_2 = torch.nn.Linear(64, 64)
+        self.linear_3 = torch.nn.Linear(64, n_output)
+
+    def forward(self, x):
+        return self.linear_3(torch.relu(self.linear_2(torch.relu(self.linear_1(x)))))
+
+
+class CartPoleAgent:
+    """A gym-style host agent: greedy discrete actions, return = summed reward."""
+
+    def __init__(self, device=torch.device("cpu")):
+        import gym
+        self.env, self.device = gym.make("CartPole-v1"), device
+
+    def rollout(self, policy, render=False):
+        observation, done, total = self.env.reset(), False, 0.0
+        with torch.no_grad():
+            while not done:
+                action = int(torch.argmax(policy(torch.from_numpy(observation).float().to(self.device))))
+                observation, reward, done, _ = self.env.step(action)
+                if render:
+                    self.env.render()
+                total += reward
+        return total
+
+
+class WalkerAgent:
+    """The novelty-search agent protocol: rollout -> (reward, behaviour characterisation), the
+    characterisation being the first and the last ``n`` actions of the episode."""
+
+    def __init__(self, device=torch.device("cpu"), n=32):
+        import gym
+        self.env, self.device, self.n = gym.make("BipedalWalker-v3"), device, n
+
+    def rollout(self, policy, render=False):
+        observation, done, total = self.env.reset(), False, 0.0
+        first, last = [], collections.deque(maxlen=self.n)
+        with torch.no_grad():
+            while not done:
+                action = policy(torch.from_numpy(observation).float().to(self.device)).cpu().numpy()
+                observation, reward, done, _ = self.env.step(action)
+                total += reward
+                last.append(action)
+                if len(first) < self.n:
+                    first.append(action)
+        return total, np.concatenate([first, last]).flatten()
+
+
+def cartpole_program(n_steps, population=8):
+    """examples/cartpole_es.py: train, then roll out es.policy and a Policy loaded from es.best_policy_dict."""
+    import estorch
+    device = torch.device("cpu")
+    agent = CartPoleAgent()
+    n_input, n_output = agent.env.observation_space.shape[0], agent.env.action_space.n
+    es = estorch.ES(Policy, CartPoleAgent, torch.optim.Adam, population_size=population, sigma=0.02, device=device,
+                    policy_kwargs={"n_input": n_input, "n_output": n_output}, agent_kwargs={"device": device},
+                    optimizer_kwargs={"lr": 0.01})
+    es.train(n_steps=n_steps, n_proc=1)
+    print(f"Latest Policy Reward: {agent.rollout(es.policy)}")
+    policy = Policy(n_input, n_output).to(device)
+    policy.load_state_dict(es.best_policy_dict)
+    print(f"Best Policy Reward: {agent.rollout(policy)}")
+    return es
+
+
+def early_stopping_program(n_steps, population=8):
+    """examples/early_stopping.py: log() reads population_returns / population_parameters and calls
+    terminate() once a member reaches CartPole's maximum of 500."""
+    import estorch
+
+    class ES(estorch.ES):
+        def log(self):
+            idx = int(np.argmax(self.population_returns[:, 0]))
+            reward = self.population_returns[idx, 0]
+            print(f"Reward: {reward}")
+            if reward == 500:
+                self.best = self.population_parameters[idx]
+                self.terminate()
+
+    device = torch.device("cpu")
+    agent = CartPoleAgent()
+    n_input, n_output = agent.env.observation_space.shape[0], agent.env.action_space.n
+    es = ES(Policy, CartPoleAgent, torch.optim.Adam, population_size=population, sigma=0.02, device=device,
+            policy_kwargs={"n_input": n_input, "n_output": n_output}, agent_kwargs={"device": device},
+            optimizer_kwargs={"lr": 0.01})
+    es.train(n_steps=n_steps, n_proc=1)
+    policy = Policy(n_input, n_output).to(device)
+    torch.nn.utils.vector_to_parameters(es.best.to(device), policy.parameters())
+    print(f"Reward: {agent.rollout(policy)}")
+    return es
+
+
+def custom_es_program(n_steps, population=8):
+    """examples/custom_es.py: a subclass overrides _sample_policy / _calculate_grad (mirrored sampling,
+    PGPE-style update) and uses the package's rank_transformation."""
+    import estorch
+
+    class SymmetricES(estorch.ES):
+        def _sample_policy(self, policy):
+            theta = torch.nn.utils.parameters_to_vector(policy.parameters()).detach().cpu()
+            epsilon = self.sigma * torch.randn(self.population_size // 2, theta.numel())
+            return torch.cat((theta + epsilon, theta - epsilon)), epsilon
+
+        def _calculate_grad(self, epsilon):
+            ranked = torch.from_numpy(estorch.rank_transformation(self.population_returns.squeeze())).float()
+            half = self.population_size // 2
+            return (ranked[:half] - ranked[half:]) @ epsilon / (half * self.sigma)
+
+    device = torch.device("cpu")
+    agent = CartPoleAgent()
+    n_input, n_output = agent.env.observation_space.shape[0], agent.env.action_space.n
+    es = SymmetricES(Policy, CartPoleAgent, torch.optim.Adam, population_size=population, sigma=0.02, device=device,
+                     policy_kwargs={"n_input": n_input, "n_output": n_output}, agent_kwargs={"device": device},
+                     optimizer_kwargs={"lr": 0.01})
+    es.train(n_steps=n_steps, n_proc=1)
+    policy = Policy(n_input, n_output).to(device)
+    policy.load_state_dict(es.best_policy_dict)
+    print(f"Best Policy Reward: {agent.rollout(policy)}")
+    return es
+
+
+def nsra_program(n_steps, population=8):
+    """examples/nsra_es.py: NSRA_ES with an adaptive weight, then roll out every meta-population member
+    and the best policy."""
+    import estorch
+    device = torch.device("cpu")
+    agent = WalkerAgent()
+    n_input, n_output = agent.env.observation_space.shape[0], agent.env.action_space.shape[0]
+    es = estorch.NSRA_ES(Policy, WalkerAgent, torch.optim.Adam, population_size=population, sigma=0.02, weight_t=10,
+                         device=device, policy_kwargs={"n_input": n_input, "n_output": n_output},
+                         agent_kwargs={"device": device}, optimizer_kwargs={"lr": 0.01})
+    es.train(n_steps=n_steps, n_proc=1)
+    for idx, (policy, _) in enumerate(es.meta_population):
+        reward, _ = agent.rollout(policy)
+        print(f"Reward of {idx}. policy from the meta population: {reward}")
+    policy = Policy(n_input, n_output).to(device)
+    policy.load_state_dict(es.best_policy_dict)
+    print(f"Best Policy Reward: {agent.rollout(policy)[0]}")
+    return es
+
+
 @pytest.fixture
 def reference_world(monkeypatch):
-    """``import estorch`` -> this package (CPU stand-in backend), ``import gym`` -> the stand-in,
-    the examples directory importable (early_stopping.py / custom_es.py import cartpole_es)."""
+    """``import estorch`` -> this package (CPU stand-in backend), ``import gym`` -> the stand-in."""
     gym = types.ModuleType("gym")
     gym.make = lambda name: CartPoleStandIn() if name.startswith("CartPole") else WalkerStandIn()
     monkeypatch.setitem(sys.modules, "gym", gym)
     monkeypatch.setitem(sys.modules, "estorch", estorch_b200)
-    monkeypatch.syspath_prepend(EXAMPLES)
-    sys.modules.pop("cartpole_es", None)
     real_init = estorch_b200.ES.__init__
 
     def init_with_cpu_backend(self, *a, **kw):
@@ -104,63 +245,44 @@ def reference_world(monkeypatch):
         kw.setdefault("noise_table_size", 1 << 16)
         real_init(self, *a, **kw)
     monkeypatch.setattr(estorch_b200.ES, "__init__", init_with_cpu_backend)
-    yield
-    sys.modules.pop("cartpole_es", None)
-
-
-def _run_example(name, n_steps, population=8):
-    src = open(os.path.join(EXAMPLES, name)).read()
-    src, n1 = re.subn(r"n_proc=\d+", "n_proc=1", src)
-    src, n2 = re.subn(r"n_steps=\d+", f"n_steps={n_steps}", src)
-    src, n3 = re.subn(r"population_size=\d+", f"population_size={population}", src)
-    assert n1 == 1 and n2 == 1 and n3 == 1, "the example's launch line changed upstream"
-    scope = {"__name__": "__main__", "__file__": os.path.join(EXAMPLES, name)}
-    exec(compile(src, os.path.join(EXAMPLES, name), "exec"), scope)
-    return scope
 
 
 def test_cartpole_example_runs_unmodified(reference_world, capsys):
-    """examples/cartpole_es.py: ES(Policy, Agent, Adam, ...).train(), then es.policy and
+    """cartpole_es.py: ES(Policy, Agent, Adam, ...).train(), then es.policy and
     es.best_policy_dict feed the user's own rollout (estorch.py:108-117 attributes)."""
-    scope = _run_example("cartpole_es.py", n_steps=2)
-    es = scope["es"]
+    es = cartpole_program(n_steps=2)
     assert type(es).__name__ == "ES" and not es._fused        # a gym-style host agent: hooks path
     assert es.step == 2 and es.population_returns.shape == (8, 1) and es.population_returns.dtype == np.float32
-    assert set(es.best_policy_dict) == set(scope["Policy"](4, 2).state_dict())
+    assert set(es.best_policy_dict) == set(Policy(4, 2).state_dict())
     out = capsys.readouterr().out
     assert "Latest Policy Reward" in out and "Best Policy Reward" in out and "Episode Reward" in out
 
 
-def test_early_stopping_example_runs_unmodified(reference_world, capsys):
-    """examples/early_stopping.py overrides log(), indexes population_parameters by member and
+def test_early_stopping_example_runs_unmodified(reference_world, capsys, monkeypatch):
+    """early_stopping.py overrides log(), indexes population_parameters by member and
     calls terminate() (estorch.py:150-152): make every episode 'perfect' so that it triggers."""
-    import cartpole_es                                            # the reference's module, via syspath
-    monkey_reward = 500.0
-    cartpole_es.Agent.rollout = lambda self, policy, render=False: monkey_reward
-    scope = _run_example("early_stopping.py", n_steps=5)
-    es = scope["es"]
+    monkeypatch.setattr(CartPoleAgent, "rollout", lambda self, policy, render=False: 500.0)
+    es = early_stopping_program(n_steps=5)
     assert es.step == 1                                            # stopped after the first generation
     assert tuple(es.best.shape) == (es.n_parameters,)
     assert "Reward: 500" in capsys.readouterr().out
 
 
 def test_custom_es_example_runs_unmodified(reference_world, capsys):
-    """examples/custom_es.py overrides _sample_policy / _calculate_grad and imports
+    """custom_es.py overrides _sample_policy / _calculate_grad and imports
     rank_transformation from the package: the engine must honour the overrides."""
-    scope = _run_example("custom_es.py", n_steps=2)
-    es = scope["es"]
+    es = custom_es_program(n_steps=2)
     assert type(es).__name__ == "SymmetricES" and not es._fused
     assert es.step == 2 and torch.isfinite(torch.nn.utils.parameters_to_vector(es.policy.parameters())).all()
     assert "Best Policy Reward" in capsys.readouterr().out
 
 
 def test_nsra_example_runs_unmodified(reference_world, capsys):
-    """examples/nsra_es.py: rollout -> (reward, behaviour characterisation), the archive /
+    """nsra_es.py: rollout -> (reward, behaviour characterisation), the archive /
     meta-population / adaptive weight of estorch.py:388-472,623-662, es.meta_population and
     es.best_policy_dict afterwards."""
     np.random.seed(0)
-    scope = _run_example("nsra_es.py", n_steps=2, population=8)
-    es = scope["es"]
+    es = nsra_program(n_steps=2, population=8)
     assert type(es).__name__ == "NSRA_ES" and len(es.meta_population) == 3
     assert es.population_returns.shape == (8, 2) and len(es._archive) == 3 + 2    # +1 behaviour per generation
     assert not hasattr(es, "policy")                                              # as in the reference (estorch.py:135-137)
